@@ -132,7 +132,10 @@ SAILOR_PT_API int32_t SailorPt_Run(const SailorPtParams* params);
 
 /* ---- staged entry points (the same pipeline, one stage per call; used by parity tests and the bench) ---- */
 
-/* Load + flatten (PathTracer.cpp:84-162, MaterialUtils.cpp:64-198) + materials/textures/lights (:164-381). */
+/* Load + flatten (PathTracer.cpp:84-162, MaterialUtils.cpp:64-198) + materials/textures/lights (:164-381).
+ * Also expands EXT_mesh_gpu_instancing (not read by the reference): a node's mesh is drawn once per instance, in the triangle
+ * order of the same scene with one child node per instance placed before the node's children.  A malformed instancing object
+ * gives SAILOR_PT_ERR_FORMAT; more than 1,431,655,765 flattened triangles give SAILOR_PT_ERR_LIMIT before any device allocation. */
 SAILOR_PT_API int32_t SailorPt_SceneLoad(const char* pathToModel, SailorPtScene** outScene);
 SAILOR_PT_API void SailorPt_SceneFree(SailorPtScene* scene);
 /* counts[0..5] = triangles, materials, textures, directional lights, cameras, BVH nodes used (0 before build) */

@@ -6,6 +6,12 @@
 // tangent generation (MaterialUtils.cpp:33-62) when the primitive has no TANGENT stream.  `vec4 * mat4` follows
 // glm's order m[j][0]*v0 + m[j][1]*v1 + m[j][2]*v2 + m[j][3]*v3 (glm/detail/type_mat4x4.inl:586-595).
 //
+// Input: the vertex streams of each source primitive once (SourceDesc), and the draws in triangle order (DrawDesc: source,
+// world matrix, material; drawStart: first output triangle of each draw).  A mesh placed by many nodes or instanced by
+// EXT_mesh_gpu_instancing is many draws of one source.  Output triangle t belongs to the last draw whose drawStart <= t.
+// FlattenBlockKernel finds that draw once for the first triangle of every kFlattenSpan, so a thread searches only the draws
+// its own span touches: none for a few large draws, a handful when 10^5 draws of small meshes share the scene.
+//
 // HBM layout produced (all 16-byte aligned for LDG.128):
 //   vtx      float4[3N]  (v0|v1|v2).xyz per triangle           -> BVH build input, 48 B / triangle
 //   centroid float4[N]   centroid.xyz, w = material index bits -> BVH build input, 16 B / triangle
@@ -17,16 +23,40 @@
 
 namespace spt
 {
-	struct PrimDesc
+	struct SourceDesc
 	{
-		float world[16];
-		uint32_t triStart;     // first output triangle
-		uint32_t triCount;
 		uint32_t vtxOffset;    // into pos (x3), nrm (x3), uv0/uv1 (x2), tan (x4): element = vertex
 		uint32_t idxOffset;    // into idx
 		uint32_t hasNrm, hasUv0, hasUv1, hasTan;
+		uint32_t pad[2];
+	};
+
+	struct DrawDesc
+	{
+		float world[16];
+		uint32_t source;       // into the SourceDesc table
 		uint32_t material;
-		uint32_t pad[3];
+		uint32_t pad[2];
+	};
+
+	constexpr uint32_t kFlattenSpan = 256;     // output triangles per entry of the block table (= threads per launch_for block)
+
+	// last draw d in [lo, hi) with drawStart[d] <= t (drawStart[lo] <= t)
+	SPT_HD uint32_t FindDraw(const uint32_t* drawStart, uint32_t lo, uint32_t hi, uint32_t t)
+	{
+		while (hi - lo > 1) { const uint32_t mid = (lo + hi) >> 1; if (drawStart[mid] <= t) lo = mid; else hi = mid; }
+		return lo;
+	}
+
+	// blockDraw[b] = the draw of output triangle min(b * kFlattenSpan, numTris - 1), for b in [0, ceil(numTris / kFlattenSpan)]
+	struct FlattenBlockKernel
+	{
+		const uint32_t* drawStart; uint32_t numDraws, numTris; uint32_t* blockDraw;
+		SPT_KERNEL_BODY void operator()(uint32_t b) const
+		{
+			const uint32_t t = b < (numTris - 1u) / kFlattenSpan + 1u ? b * kFlattenSpan : numTris - 1u;
+			blockDraw[b] = FindDraw(drawStart, 0u, numDraws, t);
+		}
 	};
 
 	SPT_HD V3 RowMul3(const float* M, V3 v, float w)
@@ -39,18 +69,18 @@ namespace spt
 
 	struct FlattenKernel
 	{
-		const PrimDesc* prims; uint32_t numPrims;
+		const DrawDesc* draws; const uint32_t* drawStart; const uint32_t* blockDraw; const SourceDesc* sources;
 		const float* pos; const float* nrm; const float* uv0; const float* uv1; const float* tan; const uint32_t* idx;
 		V4* vtx; V4* centroid; V4* shade; V2* uv2;
 
 		SPT_KERNEL_BODY void operator()(uint32_t t) const
 		{
-			// binary search: last primitive with triStart <= t
-			uint32_t lo = 0, hi = numPrims;
-			while (hi - lo > 1) { const uint32_t mid = (lo + hi) >> 1; if (prims[mid].triStart <= t) lo = mid; else hi = mid; }
-			const PrimDesc& P = prims[lo];
-			const uint32_t f = t - P.triStart;
-			const float* M = P.world;
+			const uint32_t b = t / kFlattenSpan;
+			const uint32_t d = FindDraw(drawStart, blockDraw[b], blockDraw[b + 1] + 1u, t);
+			const DrawDesc& D = draws[d];
+			const SourceDesc& P = sources[D.source];
+			const uint32_t f = t - drawStart[d];
+			const float* M = D.world;
 			uint32_t vi[3];
 			V3 lp[3], ln[3], wv[3], wn[3], wt[3], wb[3];
 			V2 uvA[3], uvB[3];
@@ -101,7 +131,7 @@ namespace spt
 				wb[0] = wb[1] = wb[2] = bt;
 			}
 			for (int k = 0; k < 3; k++) vtx[t * 3 + k] = v4(wv[k].x, wv[k].y, wv[k].z, 0.0f);
-			centroid[t] = v4(c.x, c.y, c.z, u2f(P.material));
+			centroid[t] = v4(c.x, c.y, c.z, u2f(D.material));
 			V4* s = shade + (size_t)t * 9;
 			s[0] = v4(wn[0].x, wn[0].y, wn[0].z, uvA[0].x);
 			s[1] = v4(wn[1].x, wn[1].y, wn[1].z, uvA[0].y);
@@ -109,7 +139,7 @@ namespace spt
 			s[3] = v4(wt[0].x, wt[0].y, wt[0].z, uvA[1].y);
 			s[4] = v4(wt[1].x, wt[1].y, wt[1].z, uvA[2].x);
 			s[5] = v4(wt[2].x, wt[2].y, wt[2].z, uvA[2].y);
-			s[6] = v4(wb[0].x, wb[0].y, wb[0].z, u2f(P.material));
+			s[6] = v4(wb[0].x, wb[0].y, wb[0].z, u2f(D.material));
 			s[7] = v4(wb[1].x, wb[1].y, wb[1].z, 0.0f);
 			s[8] = v4(wb[2].x, wb[2].y, wb[2].z, 0.0f);
 			for (int k = 0; k < 3; k++) uv2[t * 3 + k] = uvB[k];

@@ -7,6 +7,8 @@
 // world = node * parent in the reference's transposed-matrix convention, TRIANGLES primitives only, u8 material
 // index, texture slots deduplicated by (image, clamping, channels) in the order base / normal / metallicRoughness /
 // emissive / transmission, directional KHR_lights_punctual only (intensity = color * intensity / 683).
+// EXT_mesh_gpu_instancing (which the oracle does not read) draws a node's mesh once per instance, exactly as if the node had one
+// child node per instance, placed before its own children.
 #include "host_scene.h"
 #if defined(__unix__)
 #include <sys/mman.h>
@@ -16,6 +18,7 @@
 #endif
 #include "../../include/sailor_pt.h"
 
+#include <array>
 #include <atomic>
 #include <cmath>
 #include <thread>
@@ -347,51 +350,81 @@ namespace spt
 			std::vector<std::vector<float>> lightMatrix;
 			bool needDefault = false;              // some primitive uses the default material
 
+			int rc = SAILOR_PT_OK;                 // the first refusal (ERR_FORMAT / ERR_LIMIT) stops the traversal
+			std::string err;
+			// source index by the accessors a primitive reads (POSITION, NORMAL, TANGENT, TEXCOORD_0, TEXCOORD_1, indices): -1 when
+			// the primitive draws nothing
+			std::map<std::array<int, 6>, int> sourceOf;
+
+			bool Refuse(int code, int node, const std::string& what)
+			{
+				if (rc == SAILOR_PT_OK) { rc = code; err = "node[" + std::to_string(node) + "]: " + what; }
+				return false;
+			}
+
 			// node local matrix, reference convention = transpose of the mathematical matrix (MaterialUtils.cpp:186-191)
 			void LocalMatrix(const Json& n, float* out) const
 			{
-				float m[16];
 				const Json& jm = n.at("matrix");
-				if (jm.size() == 16) { for (int i = 0; i < 16; i++) m[i] = (float)jm.at(i).num; }
-				else
+				if (jm.size() == 16)
 				{
-					float t[3] = { 0, 0, 0 }, s[3] = { 1, 1, 1 }, q[4] = { 0, 0, 0, 1 };
-					if (n.at("translation").size() == 3) for (int i = 0; i < 3; i++) t[i] = (float)n.at("translation").at(i).num;
-					if (n.at("scale").size() == 3) for (int i = 0; i < 3; i++) s[i] = (float)n.at("scale").at(i).num;
-					if (n.at("rotation").size() == 4) for (int i = 0; i < 4; i++) q[i] = (float)n.at("rotation").at(i).num;
-					const float x = q[0], y = q[1], z = q[2], w = q[3];
-					const float R[3][3] = {
-						{ 1.0f - 2.0f * (y * y + z * z), 2.0f * (x * y - w * z), 2.0f * (x * z + w * y) },
-						{ 2.0f * (x * y + w * z), 1.0f - 2.0f * (x * x + z * z), 2.0f * (y * z - w * x) },
-						{ 2.0f * (x * z - w * y), 2.0f * (y * z + w * x), 1.0f - 2.0f * (x * x + y * y) } };
-					for (int c = 0; c < 3; c++) { for (int r = 0; r < 3; r++) m[c * 4 + r] = R[r][c] * s[c]; m[c * 4 + 3] = 0.0f; }
-					m[12] = t[0]; m[13] = t[1]; m[14] = t[2]; m[15] = 1.0f;
+					float m[16];
+					for (int i = 0; i < 16; i++) m[i] = (float)jm.at(i).num;
+					for (int c = 0; c < 4; c++) for (int r = 0; r < 4; r++) out[c * 4 + r] = m[r * 4 + c]; // transpose
+					return;
 				}
+				float t[3] = { 0, 0, 0 }, s[3] = { 1, 1, 1 }, q[4] = { 0, 0, 0, 1 };
+				if (n.at("translation").size() == 3) for (int i = 0; i < 3; i++) t[i] = (float)n.at("translation").at(i).num;
+				if (n.at("scale").size() == 3) for (int i = 0; i < 3; i++) s[i] = (float)n.at("scale").at(i).num;
+				if (n.at("rotation").size() == 4) for (int i = 0; i < 4; i++) q[i] = (float)n.at("rotation").at(i).num;
+				TrsMatrix(t, q, s, out);
+			}
+
+			// translation, rotation quaternion (x, y, z, w), scale -> matrix in the reference convention.  Node TRS and the
+			// instances of EXT_mesh_gpu_instancing both go through here, so an instance has the bits of a child node with its TRS.
+			static void TrsMatrix(const float* t, const float* q, const float* s, float* out)
+			{
+				float m[16];
+				const float x = q[0], y = q[1], z = q[2], w = q[3];
+				const float R[3][3] = {
+					{ 1.0f - 2.0f * (y * y + z * z), 2.0f * (x * y - w * z), 2.0f * (x * z + w * y) },
+					{ 2.0f * (x * y + w * z), 1.0f - 2.0f * (x * x + z * z), 2.0f * (y * z - w * x) },
+					{ 2.0f * (x * z - w * y), 2.0f * (y * z + w * x), 1.0f - 2.0f * (x * x + y * y) } };
+				for (int c = 0; c < 3; c++) { for (int r = 0; r < 3; r++) m[c * 4 + r] = R[r][c] * s[c]; m[c * 4 + 3] = 0.0f; }
+				m[12] = t[0]; m[13] = t[1]; m[14] = t[2]; m[15] = 1.0f;
 				for (int c = 0; c < 4; c++) for (int r = 0; r < 4; r++) out[c * 4 + r] = m[r * 4 + c]; // transpose
 			}
 
-			void Primitive(const Json& prim, const float* world)
+			// the streams of a primitive, read on its first use; -1 when it draws nothing (not TRIANGLES, POSITION unreadable)
+			int Source(const Json& prim)
 			{
 				const int mode = prim.at("mode").integer(4);
-				if (mode != 4) return;
+				if (mode != 4) return -1;
 				const Json& attrs = prim.at("attributes");
-				const Accessor pos = g.accessor(attrs.at("POSITION").integer(-1));
-				if (!pos.valid) return;
-				scene.prims.emplace_back();
-				HostPrimitive& hp = scene.prims.back();
+				const std::array<int, 6> key = { attrs.at("POSITION").integer(-1), attrs.at("NORMAL").integer(-1), attrs.at("TANGENT").integer(-1),
+					attrs.at("TEXCOORD_0").integer(-1), attrs.at("TEXCOORD_1").integer(-1), prim.at("indices").integer(-1) };
+				const auto found = sourceOf.find(key);
+				if (found != sourceOf.end()) return found->second;
+				int& slot = sourceOf[key];
+				slot = -1;
+				const Accessor pos = g.accessor(key[0]);
+				if (!pos.valid) return -1;
+				scene.sources.emplace_back();
+				HostSource& hp = scene.sources.back();
+				slot = (int)scene.sources.size() - 1;
 				ReadStream(pos, 3, hp.pos);
 				// an attribute stream whose element count differs from POSITION's is malformed: it is ignored (the device buffers are
 				// sized by the position count, and FlattenKernel indexes every stream with position indices)
-				auto attr = [&](const char* name) { Accessor a = g.accessor(attrs.at(name).integer(-1)); if (a.valid && a.count != pos.count) a.valid = false; return a; };
-				const Accessor nrm = attr("NORMAL");
+				auto attr = [&](int k) { Accessor a = g.accessor(key[k]); if (a.valid && a.count != pos.count) a.valid = false; return a; };
+				const Accessor nrm = attr(1);
 				if (nrm.valid) ReadStream(nrm, 3, hp.nrm);
-				const Accessor tan = attr("TANGENT");
+				const Accessor tan = attr(2);
 				if (tan.valid && tan.comps == 4) ReadStream(tan, 4, hp.tan);
-				const Accessor uv0 = attr("TEXCOORD_0");
+				const Accessor uv0 = attr(3);
 				if (uv0.valid) ReadStream(uv0, 2, hp.uv0);
-				const Accessor uv1 = attr("TEXCOORD_1");
+				const Accessor uv1 = attr(4);
 				if (uv1.valid) ReadStream(uv1, 2, hp.uv1);
-				const Accessor idx = g.accessor(prim.at("indices").integer(-1));
+				const Accessor idx = g.accessor(key[5]);
 				const size_t numIdx = idx.valid ? idx.count : pos.count;
 				const size_t faces = numIdx / 3;
 				hp.idx.resize(faces * 3);
@@ -405,21 +438,77 @@ namespace spt
 				else for (size_t i = 0; i < n3; i++) dst[i] = idx.valid ? ReadIndex(idx, i) : (uint32_t)i;
 				const uint32_t limit = (uint32_t)(pos.count < 0xFFFFFFFFull ? pos.count : 0xFFFFFFFFull);
 				for (size_t i = 0; i < n3; i++) dst[i] = dst[i] < limit ? dst[i] : 0u;      // out-of-range indices read vertex 0 (no crash on bad files)
-				memcpy(hp.world, world, sizeof(hp.world));
-				// a primitive without a material (or with an index outside the array) gets the DEFAULT material, which Assimp's glTF2
-				// importer appends after the file's own materials (index = their count); LoadGltf appends it when `needDefault` is set
+				return slot;
+			}
+
+			// a primitive without a material (or with an index outside the array) gets the DEFAULT material, which Assimp's glTF2
+			// importer appends after the file's own materials (index = their count); LoadGltf appends it when `needDefault` is set
+			uint32_t Material(const Json& prim)
+			{
 				const int mat = prim.at("material").integer(-1);
 				const size_t nm = g.root.at("materials").size();
 				const bool own = mat >= 0 && (size_t)mat < nm;
 				if (!own) needDefault = true;
-				hp.material = (uint32_t)(own ? (size_t)mat : nm);
-				scene.numTriangles += faces;
+				return (uint32_t)(own ? (size_t)mat : nm);
+			}
+
+			// draws every primitive of a mesh once per world matrix (one matrix: an ordinary node; K: the node's instances), instance-major
+			void DrawMesh(const Json& prims, const std::vector<int>& src, const float* worlds, size_t count)
+			{
+				for (size_t k = 0; k < count; k++)
+					for (size_t i = 0; i < prims.size(); i++)
+					{
+						if (src[i] < 0) continue;
+						const uint32_t material = Material(prims.at(i));
+						const uint64_t faces = scene.sources[(size_t)src[i]].idx.size() / 3;
+						if (!faces) continue;
+						scene.draws.emplace_back();
+						HostDraw& d = scene.draws.back();
+						d.source = (uint32_t)src[i]; d.material = material;
+						memcpy(d.world, worlds + k * 16, sizeof(d.world));
+						scene.numTriangles += faces;
+					}
+			}
+
+			// EXT_mesh_gpu_instancing: the world matrix of every instance, TRS_i * nodeWorld (a child node with that TRS)
+			bool InstanceMatrices(const Json& attrs, int node, const float* world, uint64_t meshFaces, std::vector<float>& out)
+			{
+				struct Attr { const char* name; int comps; Accessor a; bool present; } A[3] = { { "TRANSLATION", 3, {}, false }, { "ROTATION", 4, {}, false }, { "SCALE", 3, {}, false } };
+				size_t count = 0; bool any = false;
+				for (Attr& at : A)
+				{
+					const Json* j = attrs.find(at.name);
+					if (!j) continue;
+					at.present = true;
+					at.a = g.accessor(j->isNumber() ? j->integer(-1) : -1);
+					if (!at.a.valid) return Refuse(SAILOR_PT_ERR_FORMAT, node, std::string("EXT_mesh_gpu_instancing: the ") + at.name + " accessor is missing or unreadable");
+					if (at.a.comps != at.comps) return Refuse(SAILOR_PT_ERR_FORMAT, node, std::string("EXT_mesh_gpu_instancing: ") + at.name + (at.comps == 3 ? " is not VEC3" : " is not VEC4"));
+					if (any && at.a.count != count) return Refuse(SAILOR_PT_ERR_FORMAT, node, "EXT_mesh_gpu_instancing: the attributes have different counts");
+					count = at.a.count; any = true;
+				}
+				// names starting with '_' are application-specific and ignored (the extension's specification); nothing else is defined
+				if (!any) return Refuse(SAILOR_PT_ERR_FORMAT, node, "EXT_mesh_gpu_instancing: no TRANSLATION, ROTATION or SCALE attribute");
+				// the expanded triangle count in 64 bits, before any per-instance data exists
+				if (meshFaces && (uint64_t)count > (kMaxTriangles - scene.numTriangles) / meshFaces)
+					return Refuse(SAILOR_PT_ERR_LIMIT, node, "EXT_mesh_gpu_instancing: " + std::to_string(count) + " instances of " + std::to_string(meshFaces) +
+						" triangles exceed the " + std::to_string(kMaxTriangles) + " triangles a scene may have");
+				out.resize(count * 16);
+				for (size_t i = 0; i < count; i++)
+				{
+					float t[3] = { 0, 0, 0 }, q[4] = { 0, 0, 0, 1 }, s[3] = { 1, 1, 1 }, local[16];
+					if (A[0].present) for (int c = 0; c < 3; c++) t[c] = ReadFloat(A[0].a, i, c);
+					if (A[1].present) for (int c = 0; c < 4; c++) q[c] = ReadFloat(A[1].a, i, c);
+					if (A[2].present) for (int c = 0; c < 3; c++) s[c] = ReadFloat(A[2].a, i, c);
+					TrsMatrix(t, q, s, local);
+					Mat4Mul(local, world, out.data() + i * 16);
+				}
+				return true;
 			}
 
 			void Node(int index, const float* parent, int depth)
 			{
 				const Json& nodes = g.root.at("nodes");
-				if (index < 0 || (size_t)index >= nodes.size() || depth > 512) return;
+				if (rc != SAILOR_PT_OK || index < 0 || (size_t)index >= nodes.size() || depth > 512) return;
 				const Json& n = nodes.at(index);
 				float local[16], world[16];
 				LocalMatrix(n, local);
@@ -428,7 +517,21 @@ namespace spt
 				if (mesh >= 0 && (size_t)mesh < g.root.at("meshes").size())
 				{
 					const Json& prims = g.root.at("meshes").at(mesh).at("primitives");
-					for (size_t i = 0; i < prims.size(); i++) Primitive(prims.at(i), world);
+					std::vector<int> src(prims.size());
+					uint64_t faces = 0;
+					for (size_t i = 0; i < prims.size(); i++) { src[i] = Source(prims.at(i)); if (src[i] >= 0) faces += scene.sources[(size_t)src[i]].idx.size() / 3; }
+					const Json* inst = n.at("extensions").find("EXT_mesh_gpu_instancing");
+					if (inst && inst->find("attributes"))
+					{
+						std::vector<float> worlds;
+						if (!InstanceMatrices(inst->at("attributes"), index, world, faces, worlds)) return;
+						DrawMesh(prims, src, worlds.data(), worlds.size() / 16);
+					}
+					else
+					{
+						if (faces > kMaxTriangles - scene.numTriangles) { Refuse(SAILOR_PT_ERR_LIMIT, index, "the scene has more than " + std::to_string(kMaxTriangles) + " triangles"); return; }
+						DrawMesh(prims, src, world, 1);
+					}
 				}
 				const int cam = n.at("camera").integer(-1);
 				if (cam >= 0 && (size_t)cam < scene.cameras.size() && !cameraSeen[cam])
@@ -602,6 +705,7 @@ namespace spt
 		const int sceneIndex = g.root.at("scene").integer(0);
 		const Json& roots = g.root.at("scenes").at(sceneIndex >= 0 ? sceneIndex : 0).at("nodes");
 		for (size_t i = 0; i < roots.size(); i++) b.Node(roots.at(i).integer(-1), identity, 0);
+		if (b.rc != SAILOR_PT_OK) { err = b.err; return b.rc; }
 		for (size_t i = 0; i < scene.cameras.size(); i++) if (!b.cameraSeen[i]) scene.cameras[i].name.clear();
 
 		// images are decoded lazily, once per texture slot

@@ -1,8 +1,8 @@
 // host_scene.h — what the glTF front end hands to the device pipeline (host memory, product code).
 //
-// This is the input side of the hot path (SURVEY §8 rows a10/a11/a12/a14): raw per-primitive vertex streams and a
-// world matrix per primitive (flattened on the DEVICE by flatten.cuh), material factors, RGBA8 texels (converted to
-// float texels on the device), cameras and directional lights.  Loader contract: DESIGN.md "loader contract".
+// This is the input side of the hot path (SURVEY §8 rows a10/a11/a12/a14): raw vertex streams, once per source primitive,
+// and a draw table of (source, world matrix, material) (flattened on the DEVICE by flatten.cuh), material factors, RGBA8
+// texels (converted to float texels on the device), cameras and directional lights.  Loader contract: DESIGN.md "loader contract".
 #pragma once
 #include <stdint.h>
 #include <string>
@@ -27,7 +27,9 @@ namespace spt
 	};
 	static_assert(sizeof(MaterialGpu) == 144, "MaterialGpu layout");
 
-	struct HostPrimitive
+	// The vertex streams of one glTF primitive, read once per document: every node that reaches a primitive with the same
+	// accessors, and every instance of EXT_mesh_gpu_instancing, draws these streams again without copying them.
+	struct HostSource
 	{
 		std::vector<float> pos;     // 3 per vertex
 		std::vector<float> nrm;     // 3 per vertex or empty (-> flat face normals, aiProcess_GenNormals)
@@ -35,9 +37,22 @@ namespace spt
 		std::vector<float> uv1;     // 2 per vertex or empty
 		std::vector<float> tan;     // 4 per vertex or empty
 		std::vector<uint32_t> idx;  // 3 per triangle (identity when the primitive is not indexed)
-		float world[16];            // reference convention: memory = row-major world matrix (glm m[c][r] = world[c*4+r])
-		uint32_t material = 0;      // already truncated to u8 like Triangle::m_materialIndex (Bounds.h:21)
 	};
+
+	// One placement of a source in the flattened scene.  Draws are in the scene's triangle order: the flattened triangles are
+	// the triangles of each draw's source, draw after draw.
+	struct HostDraw
+	{
+		uint32_t source = 0;        // into HostScene::sources
+		uint32_t material = 0;      // already truncated to u8 like Triangle::m_materialIndex (Bounds.h:21)
+		float world[16];            // reference convention: memory = row-major world matrix (glm m[c][r] = world[c*4+r])
+	};
+
+	// Most flattened triangles a scene may have.  The device pipeline indexes triangles with 32-bit integers, and the largest
+	// product it forms from a triangle index is t * 3 + 2 (vertex slots of flatten, BVH build and every traversal layout);
+	// node indices stay below 2 N and leaf references below 2^31 (traverse.cuh kLeafBit).  floor((2^32 - 1) / 3) keeps all of
+	// them exact.  Device memory runs out long before this (about 232 B per flattened triangle plus the BVH).
+	constexpr uint64_t kMaxTriangles = 0xFFFFFFFFull / 3u;
 
 	struct HostTexture
 	{
@@ -53,7 +68,7 @@ namespace spt
 	struct HostCamera
 	{
 		std::string name;
-		float matrix[16];           // reference convention (see HostPrimitive::world)
+		float matrix[16];           // reference convention (see HostDraw::world)
 		float aspect = 0.0f;
 		float hFov = 0.0f;
 	};
@@ -62,12 +77,13 @@ namespace spt
 
 	struct HostScene
 	{
-		std::vector<HostPrimitive> prims;
+		std::vector<HostSource> sources;
+		std::vector<HostDraw> draws;
 		std::vector<MaterialGpu> materials;
 		std::vector<HostTexture> textures;
 		std::vector<HostCamera> cameras;
 		std::vector<HostLight> lights;
-		uint64_t numTriangles = 0;
+		uint64_t numTriangles = 0;  // flattened (all draws), at most kMaxTriangles
 		// which kernel traces this scene's secondary rays fastest (0 unknown; render.cuh decides it with a timed probe on the first frame): kept with the
 		// parsed file so that reloads served by the scene cache and the per-device replicas of a multi-device render do not probe again
 		mutable uint32_t traversalChoice = 0;

@@ -157,54 +157,71 @@ namespace spt
 		int Upload()
 		{
 			const double t0 = HostNow();
-			numTris = (uint32_t)Host().numTriangles;
+			const HostScene& H = Host();
+			if (H.numTriangles > kMaxTriangles) { ctx.error = "the scene has more than " + std::to_string(kMaxTriangles) + " triangles"; return SAILOR_PT_ERR_LIMIT; }
+			numTris = (uint32_t)H.numTriangles;
 			counter.Alloc(ctx, 16); counter.Zero(ctx);
 			if (numTris == 0) return CudaStatus();
-			// The primitive streams go to the device piece by piece, straight from the importer's vectors (no host-side concatenation:
-			// at 10 M triangles that was hundreds of MB of extra copies).  A stream a primitive lacks is never read (FlattenKernel
-			// looks at PrimDesc::has*), so its part of the device buffer stays uninitialised.
-			std::vector<PrimDesc> descs(Host().prims.size());
-			uint32_t triStart = 0, vtxOffset = 0, idxOffset = 0;
+			// Each source primitive's streams go to the device once, however many draws place it.  With few sources they are copied
+			// piece by piece, straight from the importer's vectors (no host-side concatenation: at 10 M triangles that was hundreds of
+			// MB of extra copies).  A stream a source lacks is never read (FlattenKernel looks at SourceDesc::has*), so its part of
+			// the device buffer stays uninitialised.
+			std::vector<SourceDesc> srcs(H.sources.size());
+			uint64_t vtxTotal = 0, idxTotal = 0;
 			bool anyNrm = false, anyUv0 = false, anyUv1 = false, anyTan = false;
-			for (size_t i = 0; i < Host().prims.size(); i++)
+			for (size_t i = 0; i < H.sources.size(); i++)
 			{
-				const HostPrimitive& hp = Host().prims[i];
-				PrimDesc& d = descs[i];
+				const HostSource& hs = H.sources[i];
+				SourceDesc& d = srcs[i];
 				memset(&d, 0, sizeof(d));
-				memcpy(d.world, hp.world, sizeof(d.world));
-				const uint32_t nv = (uint32_t)(hp.pos.size() / 3);
-				d.triStart = triStart; d.triCount = (uint32_t)(hp.idx.size() / 3);
-				d.vtxOffset = vtxOffset; d.idxOffset = idxOffset;
-				d.hasNrm = !hp.nrm.empty(); d.hasUv0 = !hp.uv0.empty(); d.hasUv1 = !hp.uv1.empty(); d.hasTan = !hp.tan.empty();
+				d.vtxOffset = (uint32_t)vtxTotal; d.idxOffset = (uint32_t)idxTotal;
+				d.hasNrm = !hs.nrm.empty(); d.hasUv0 = !hs.uv0.empty(); d.hasUv1 = !hs.uv1.empty(); d.hasTan = !hs.tan.empty();
 				anyNrm |= d.hasNrm != 0; anyUv0 |= d.hasUv0 != 0; anyUv1 |= d.hasUv1 != 0; anyTan |= d.hasTan != 0;
-				d.material = hp.material;
-				triStart += d.triCount; vtxOffset += nv; idxOffset += (uint32_t)hp.idx.size();
+				vtxTotal += hs.pos.size() / 3; idxTotal += hs.idx.size();
 			}
-			// empty primitives would break the binary search in FlattenKernel: drop them
-			std::vector<PrimDesc> live;
-			for (const auto& d : descs) if (d.triCount) live.push_back(d);
+			// FlattenKernel forms vertex * 4 (tangents) and index offsets in 32 bits
+			if (vtxTotal > 0xFFFFFFFFull / 4u || idxTotal > 0xFFFFFFFFull) { ctx.error = "the scene's vertex streams are too large for 32-bit offsets"; return SAILOR_PT_ERR_LIMIT; }
+			const uint32_t vtxOffset = (uint32_t)vtxTotal, idxOffset = (uint32_t)idxTotal;
+			std::vector<DrawDesc> draws(H.draws.size());
+			std::vector<uint32_t> drawStart(H.draws.size() + 1);
+			uint64_t triStart = 0;
+			for (size_t i = 0; i < H.draws.size(); i++)
+			{
+				const HostDraw& hd = H.draws[i];
+				DrawDesc& d = draws[i];
+				memset(&d, 0, sizeof(d));
+				memcpy(d.world, hd.world, sizeof(d.world));
+				d.source = hd.source; d.material = hd.material;
+				drawStart[i] = (uint32_t)triStart;
+				triStart += H.sources[hd.source].idx.size() / 3;
+			}
+			drawStart[H.draws.size()] = (uint32_t)triStart;
+			if (triStart != numTris) { ctx.error = "draw table does not cover the scene's triangles"; return SAILOR_PT_ERR_FORMAT; }
 
-			DevBuf<PrimDesc> dPrims; DevBuf<float> dPos, dNrm, dUv0, dUv1, dTan; DevBuf<uint32_t> dIdx;
-			dPrims.Upload(ctx, live);
+			DevBuf<SourceDesc> dSrcs; DevBuf<DrawDesc> dDraws; DevBuf<uint32_t> dDrawStart, dBlockDraw;
+			DevBuf<float> dPos, dNrm, dUv0, dUv1, dTan; DevBuf<uint32_t> dIdx;
+			dSrcs.Upload(ctx, srcs); dDraws.Upload(ctx, draws); dDrawStart.Upload(ctx, drawStart);
+			const uint32_t numBlocks = (numTris - 1u) / kFlattenSpan + 1u;
+			dBlockDraw.Alloc(ctx, (size_t)numBlocks + 1);
 			dPos.Alloc(ctx, (size_t)vtxOffset * 3 + 1); dIdx.Alloc(ctx, (size_t)idxOffset + 1);
 			dNrm.Alloc(ctx, anyNrm ? (size_t)vtxOffset * 3 : 1); dUv0.Alloc(ctx, anyUv0 ? (size_t)vtxOffset * 2 : 1);
 			dUv1.Alloc(ctx, anyUv1 ? (size_t)vtxOffset * 2 : 1); dTan.Alloc(ctx, anyTan ? (size_t)vtxOffset * 4 : 1);
 			if (!ctx.ok) return CudaStatus();
-			if (Host().prims.size() > 32)
+			if (H.sources.size() > 32)
 			{
-				// many small primitives: one copy per stream from a host-side concatenation beats thousands of tiny transfers
+				// many small sources: one copy per stream from a host-side concatenation beats thousands of tiny transfers
 				std::vector<float> pos((size_t)vtxOffset * 3), nrm(anyNrm ? (size_t)vtxOffset * 3 : 0), uv0(anyUv0 ? (size_t)vtxOffset * 2 : 0), uv1(anyUv1 ? (size_t)vtxOffset * 2 : 0), tan(anyTan ? (size_t)vtxOffset * 4 : 0);
 				std::vector<uint32_t> idx(idxOffset);
-				for (size_t i = 0; i < Host().prims.size(); i++)
+				for (size_t i = 0; i < H.sources.size(); i++)
 				{
-					const HostPrimitive& hp = Host().prims[i];
-					const PrimDesc& d = descs[i];
-					if (!hp.pos.empty()) memcpy(pos.data() + (size_t)d.vtxOffset * 3, hp.pos.data(), hp.pos.size() * sizeof(float));
-					if (!hp.idx.empty()) memcpy(idx.data() + d.idxOffset, hp.idx.data(), hp.idx.size() * sizeof(uint32_t));
-					if (d.hasNrm) memcpy(nrm.data() + (size_t)d.vtxOffset * 3, hp.nrm.data(), hp.nrm.size() * sizeof(float));
-					if (d.hasUv0) memcpy(uv0.data() + (size_t)d.vtxOffset * 2, hp.uv0.data(), hp.uv0.size() * sizeof(float));
-					if (d.hasUv1) memcpy(uv1.data() + (size_t)d.vtxOffset * 2, hp.uv1.data(), hp.uv1.size() * sizeof(float));
-					if (d.hasTan) memcpy(tan.data() + (size_t)d.vtxOffset * 4, hp.tan.data(), hp.tan.size() * sizeof(float));
+					const HostSource& hs = H.sources[i];
+					const SourceDesc& d = srcs[i];
+					if (!hs.pos.empty()) memcpy(pos.data() + (size_t)d.vtxOffset * 3, hs.pos.data(), hs.pos.size() * sizeof(float));
+					if (!hs.idx.empty()) memcpy(idx.data() + d.idxOffset, hs.idx.data(), hs.idx.size() * sizeof(uint32_t));
+					if (d.hasNrm) memcpy(nrm.data() + (size_t)d.vtxOffset * 3, hs.nrm.data(), hs.nrm.size() * sizeof(float));
+					if (d.hasUv0) memcpy(uv0.data() + (size_t)d.vtxOffset * 2, hs.uv0.data(), hs.uv0.size() * sizeof(float));
+					if (d.hasUv1) memcpy(uv1.data() + (size_t)d.vtxOffset * 2, hs.uv1.data(), hs.uv1.size() * sizeof(float));
+					if (d.hasTan) memcpy(tan.data() + (size_t)d.vtxOffset * 4, hs.tan.data(), hs.tan.size() * sizeof(float));
 				}
 				if (!pos.empty()) DevUpload(ctx, dPos.p, pos.data(), pos.size() * sizeof(float));
 				if (!idx.empty()) DevUpload(ctx, dIdx.p, idx.data(), idx.size() * sizeof(uint32_t));
@@ -214,23 +231,24 @@ namespace spt
 				if (!tan.empty()) DevUpload(ctx, dTan.p, tan.data(), tan.size() * sizeof(float));
 				ctx.Sync();                                   // the staging vectors die at the end of this block
 			}
-			else for (size_t i = 0; i < Host().prims.size(); i++)
+			else for (size_t i = 0; i < H.sources.size(); i++)
 			{
-				const HostPrimitive& hp = Host().prims[i];
-				const PrimDesc& d = descs[i];
-				if (!hp.pos.empty()) DevUpload(ctx, dPos.p + (size_t)d.vtxOffset * 3, hp.pos.data(), hp.pos.size() * sizeof(float));
-				if (!hp.idx.empty()) DevUpload(ctx, dIdx.p + d.idxOffset, hp.idx.data(), hp.idx.size() * sizeof(uint32_t));
-				if (d.hasNrm) DevUpload(ctx, dNrm.p + (size_t)d.vtxOffset * 3, hp.nrm.data(), hp.nrm.size() * sizeof(float));
-				if (d.hasUv0) DevUpload(ctx, dUv0.p + (size_t)d.vtxOffset * 2, hp.uv0.data(), hp.uv0.size() * sizeof(float));
-				if (d.hasUv1) DevUpload(ctx, dUv1.p + (size_t)d.vtxOffset * 2, hp.uv1.data(), hp.uv1.size() * sizeof(float));
-				if (d.hasTan) DevUpload(ctx, dTan.p + (size_t)d.vtxOffset * 4, hp.tan.data(), hp.tan.size() * sizeof(float));
+				const HostSource& hs = H.sources[i];
+				const SourceDesc& d = srcs[i];
+				if (!hs.pos.empty()) DevUpload(ctx, dPos.p + (size_t)d.vtxOffset * 3, hs.pos.data(), hs.pos.size() * sizeof(float));
+				if (!hs.idx.empty()) DevUpload(ctx, dIdx.p + d.idxOffset, hs.idx.data(), hs.idx.size() * sizeof(uint32_t));
+				if (d.hasNrm) DevUpload(ctx, dNrm.p + (size_t)d.vtxOffset * 3, hs.nrm.data(), hs.nrm.size() * sizeof(float));
+				if (d.hasUv0) DevUpload(ctx, dUv0.p + (size_t)d.vtxOffset * 2, hs.uv0.data(), hs.uv0.size() * sizeof(float));
+				if (d.hasUv1) DevUpload(ctx, dUv1.p + (size_t)d.vtxOffset * 2, hs.uv1.data(), hs.uv1.size() * sizeof(float));
+				if (d.hasTan) DevUpload(ctx, dTan.p + (size_t)d.vtxOffset * 4, hs.tan.data(), hs.tan.size() * sizeof(float));
 			}
 			vtx.Alloc(ctx, (size_t)numTris * 3); centroid.Alloc(ctx, numTris); shade.Alloc(ctx, (size_t)numTris * 9); uv2.Alloc(ctx, (size_t)numTris * 3);
 			if (!ctx.ok) return CudaStatus();
 
 			ctx.TimerStart();
+			launch_for(ctx, numBlocks + 1u, FlattenBlockKernel{ dDrawStart.p, (uint32_t)draws.size(), numTris, dBlockDraw.p });
 			FlattenKernel fk;
-			fk.prims = dPrims.p; fk.numPrims = (uint32_t)live.size();
+			fk.draws = dDraws.p; fk.drawStart = dDrawStart.p; fk.blockDraw = dBlockDraw.p; fk.sources = dSrcs.p;
 			fk.pos = dPos.p; fk.nrm = dNrm.p; fk.uv0 = dUv0.p; fk.uv1 = dUv1.p; fk.tan = dTan.p; fk.idx = dIdx.p;
 			fk.vtx = vtx.p; fk.centroid = centroid.p; fk.shade = shade.p; fk.uv2 = uv2.p;
 			launch_for(ctx, numTris, fk);
