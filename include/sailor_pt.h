@@ -135,7 +135,11 @@ SAILOR_PT_API int32_t SailorPt_Run(const SailorPtParams* params);
 /* Load + flatten (PathTracer.cpp:84-162, MaterialUtils.cpp:64-198) + materials/textures/lights (:164-381).
  * Also expands EXT_mesh_gpu_instancing (not read by the reference): a node's mesh is drawn once per instance, in the triangle
  * order of the same scene with one child node per instance placed before the node's children.  A malformed instancing object
- * gives SAILOR_PT_ERR_FORMAT; more than 1,431,655,765 flattened triangles give SAILOR_PT_ERR_LIMIT before any device allocation. */
+ * gives SAILOR_PT_ERR_FORMAT; more than 1,431,655,765 flattened triangles give SAILOR_PT_ERR_LIMIT before any device allocation.
+ * TRIANGLES, TRIANGLE_STRIP and TRIANGLE_FAN primitives draw (strip and fan corners per glTF 2.0 3.7.2.1); sparse accessors are
+ * applied (a malformed sparse block makes its accessor unreadable); quantized streams (KHR_mesh_quantization) are decoded on the
+ * device.  A primitive above the triangle limit, or a scene above 1,073,741,823 vertices, gives SAILOR_PT_ERR_LIMIT before anything
+ * is sized by that count. */
 SAILOR_PT_API int32_t SailorPt_SceneLoad(const char* pathToModel, SailorPtScene** outScene);
 SAILOR_PT_API void SailorPt_SceneFree(SailorPtScene* scene);
 /* counts[0..5] = triangles, materials, textures, directional lights, cameras, BVH nodes used (0 before build) */

@@ -59,6 +59,68 @@ namespace spt
 		}
 	};
 
+	// ---- stored streams -> the float streams and u32 triples FlattenKernel reads (before it, in the same stream) ----
+	// Sources whose streams are not float32 of FlattenKernel's width, and whose indices are not a u32 TRIANGLES list, are uploaded
+	// as the file stores them (each piece starting at a multiple of 4 bytes) and expanded here: one launch per stream kind across
+	// all such sources, each thread finding its source in a prefix table (FindDraw) as FlattenKernel finds its draw.
+
+	struct StreamDecodeDesc
+	{
+		uint64_t srcByte;      // into the staged bytes of this stream kind
+		uint32_t dstVertex;    // SourceDesc::vtxOffset
+		uint32_t componentType, comps, normalized;
+		uint32_t pad[2];
+	};
+
+	// vertex i of the decoded sources of one stream kind -> `width` floats; components beyond the stored ones read 0
+	struct DecodeStreamKernel
+	{
+		const uint32_t* start; const StreamDecodeDesc* desc; uint32_t numDesc, width; const uint8_t* src; float* dst;
+		SPT_KERNEL_BODY void operator()(uint32_t i) const
+		{
+			const uint32_t j = FindDraw(start, 0u, numDesc, i);
+			const StreamDecodeDesc& D = desc[j];
+			const uint32_t v = i - start[j];
+			const uint32_t elemBytes = D.comps * (D.componentType == 5126 || D.componentType == 5125 ? 4u : (D.componentType == 5122 || D.componentType == 5123 ? 2u : 1u));
+			const uint8_t* e = src + D.srcByte + (size_t)v * elemBytes;
+			float* o = dst + ((size_t)D.dstVertex + v) * width;
+			for (uint32_t c = 0; c < width; c++) o[c] = c < D.comps ? DecodeComponent(e, D.componentType, D.normalized != 0, c) : 0.0f;
+		}
+	};
+
+	struct IndexAssemblyDesc
+	{
+		uint64_t srcByte;      // into the staged index bytes (unused when idxType is 0)
+		uint32_t dstIndex;     // SourceDesc::idxOffset
+		uint32_t idxType;      // 0: not indexed, corner k is vertex k
+		uint32_t mode;         // 4 TRIANGLES, 5 TRIANGLE_STRIP, 6 TRIANGLE_FAN
+		uint32_t numVerts;     // an index at or above it reads vertex 0
+		uint32_t pad[2];
+	};
+
+	// face f of the assembled sources -> its three vertex indices, corners as glTF 2.0 §3.7.2.1 orders them:
+	// list (3f, 3f+1, 3f+2), strip (f, f+1+f%2, f+2-f%2), fan (f+1, f+2, 0)
+	struct AssembleIndexKernel
+	{
+		const uint32_t* start; const IndexAssemblyDesc* desc; uint32_t numDesc; const uint8_t* src; uint32_t* idx;
+		SPT_KERNEL_BODY void operator()(uint32_t t) const
+		{
+			const uint32_t j = FindDraw(start, 0u, numDesc, t);
+			const IndexAssemblyDesc& D = desc[j];
+			const uint32_t f = t - start[j];
+			uint32_t corner[3];
+			if (D.mode == 5) { corner[0] = f; corner[1] = f + 1u + (f & 1u); corner[2] = f + 2u - (f & 1u); }
+			else if (D.mode == 6) { corner[0] = f + 1u; corner[1] = f + 2u; corner[2] = 0u; }
+			else { corner[0] = f * 3u; corner[1] = f * 3u + 1u; corner[2] = f * 3u + 2u; }
+			const uint8_t* s = src + D.srcByte;
+			for (int k = 0; k < 3; k++)
+			{
+				const uint32_t v = D.idxType ? IndexAt(s, D.idxType, corner[k]) : corner[k];
+				idx[(size_t)D.dstIndex + (size_t)f * 3 + k] = v < D.numVerts ? v : 0u;
+			}
+		}
+	};
+
 	SPT_HD V3 RowMul3(const float* M, V3 v, float w)
 	{
 		return v3(M[0] * v.x + M[1] * v.y + M[2] * v.z + M[3] * w,

@@ -4,12 +4,15 @@
 // MaterialUtils.cpp:64-198 for which mesh fields are consumed).  It only PARSES: vertex streams are handed to the
 // device untransformed (flatten.cuh does the per-triangle arithmetic), texels stay RGBA8 (texture_convert kernel).
 // Loader contract (shared with the oracle's restated driver, DESIGN.md): default scene, depth-first node order,
-// world = node * parent in the reference's transposed-matrix convention, TRIANGLES primitives only, u8 material
+// world = node * parent in the reference's transposed-matrix convention, TRIANGLES primitives only (the oracle's side), u8 material
 // index, texture slots deduplicated by (image, clamping, channels) in the order base / normal / metallicRoughness /
 // emissive / transmission, directional KHR_lights_punctual only (intensity = color * intensity / 683).
 // EXT_mesh_gpu_instancing (which the oracle does not read) draws a node's mesh once per instance, exactly as if the node had one
-// child node per instance, placed before its own children.
+// child node per instance, placed before its own children.  TRIANGLE_STRIP / TRIANGLE_FAN primitives and sparse accessors (which the
+// oracle does not read either) are imported as their float32 TRIANGLES-list twin: streams stay in their stored form and are decoded
+// and assembled on the device (flatten.cuh).
 #include "host_scene.h"
+#include "hd.h"
 #if defined(__unix__)
 #include <sys/mman.h>
 #include <sys/stat.h>
@@ -28,6 +31,8 @@
 #include <limits>
 #include <map>
 #include <memory>
+#include <new>
+#include <stdexcept>
 
 namespace spt
 {
@@ -241,12 +246,17 @@ namespace spt
 			memcpy(R, tmp, sizeof(tmp));
 		}
 
+		// A readable accessor: `count` elements of `elem` bytes at base + i * stride (base null: zeros), then element sparseAt[k]
+		// replaced by the k-th element of sparseValues for k < sparseCount (sparseAt strictly increasing).  Nothing is copied here:
+		// whatever is sized by `count` is allocated by the caller, after the count has passed the caller's limit.
 		struct Accessor
 		{
 			const uint8_t* base = nullptr;
-			size_t stride = 0, count = 0;
+			size_t stride = 0, count = 0, elem = 0;
 			int componentType = 0, comps = 0;
 			bool normalized = false, valid = false;
+			const uint8_t* sparseAt = nullptr; const uint8_t* sparseValues = nullptr;
+			size_t sparseCount = 0; int sparseType = 0;
 		};
 
 		int CompsOf(const std::string& t)
@@ -273,71 +283,121 @@ namespace spt
 			std::vector<Buffer> buffers;
 			std::string baseDir;
 
+			// An accessor with a bufferView reads it; one without reads zeros, and only when it has a sparse block.  A malformed sparse
+			// block makes the accessor unreadable.
 			Accessor accessor(int index) const
 			{
 				Accessor a;
 				const Json& accs = root.at("accessors");
 				if (index < 0 || (size_t)index >= accs.size()) return a;
 				const Json& acc = accs.at(index);
+				const Json* sparse = acc.find("sparse");
+				const bool hasView = acc.find("bufferView") || !sparse;
 				const int bv = acc.at("bufferView").integer(-1);
 				const Json& views = root.at("bufferViews");
-				if (bv < 0 || (size_t)bv >= views.size()) return a;
-				const Json& view = views.at(bv);
+				if (hasView && (bv < 0 || (size_t)bv >= views.size())) return a;
+				static const Json none;
+				const Json& view = hasView ? views.at(bv) : none;
 				const int bi = view.at("buffer").integer(-1);
-				if (bi < 0 || (size_t)bi >= buffers.size()) return a;
+				if (hasView && (bi < 0 || (size_t)bi >= buffers.size())) return a;
 				a.comps = CompsOf(acc.at("type").str);
 				a.componentType = acc.at("componentType").integer(0);
-				const size_t elem = (size_t)CompSize(a.componentType) * a.comps;
+				a.elem = (size_t)CompSize(a.componentType) * a.comps;
 				// sizes and offsets come from the file: negative or absurd numbers are rejected before any size_t arithmetic, and the
 				// range check is written so that it cannot wrap
-				const double lim = 1e15;
 				const double dbs = view.at("byteStride").number(0), dvo = view.at("byteOffset").number(0), dao = acc.at("byteOffset").number(0), dcount = acc.at("count").number(0);
-				if (!(dbs >= 0 && dbs <= 65536.0 && dvo >= 0 && dvo < lim && dao >= 0 && dao < lim && dcount >= 0 && dcount < lim)) return a;
+				if (!(dbs >= 0 && dbs <= 65536.0 && dvo >= 0 && dvo < kLim && dao >= 0 && dao < kLim && dcount >= 0 && dcount < kLim)) return a;
 				const size_t bs = (size_t)dbs;
-				a.stride = bs ? bs : elem;
+				a.stride = bs ? bs : a.elem;
 				const size_t off = (size_t)dvo + (size_t)dao;
 				a.count = (size_t)dcount;
 				a.normalized = acc.at("normalized").type == Json::Bool && acc.at("normalized").b;
-				if (!elem || !a.count) return a;
-				const size_t size = buffers[bi].size();
-				if (off > size || elem > size - off || a.stride == 0 || (a.count - 1) > (size - off - elem) / a.stride) return a;
-				a.base = buffers[bi].data() + off;
+				if (!a.elem || !a.count) return a;
+				if (hasView)
+				{
+					const size_t size = buffers[bi].size();
+					if (off > size || a.elem > size - off || a.stride == 0 || (a.count - 1) > (size - off - a.elem) / a.stride) return a;
+					a.base = buffers[bi].data() + off;
+				}
+				if (sparse && !Sparse(*sparse, a)) return a;
 				a.valid = true;
 				return a;
 			}
+
+			static constexpr double kLim = 1e15;
+
+			// `bytes` bytes at o.byteOffset inside the bufferView o.bufferView, or null when they are not all inside it and its buffer
+			const uint8_t* ViewBytes(const Json& o, size_t bytes) const
+			{
+				const Json& views = root.at("bufferViews");
+				const int bv = o.at("bufferView").integer(-1);
+				if (bv < 0 || (size_t)bv >= views.size()) return nullptr;
+				const Json& view = views.at(bv);
+				const int bi = view.at("buffer").integer(-1);
+				if (bi < 0 || (size_t)bi >= buffers.size()) return nullptr;
+				const double dvo = view.at("byteOffset").number(0), dlen = view.at("byteLength").number(0), doo = o.at("byteOffset").number(0);
+				if (!(dvo >= 0 && dvo < kLim && dlen >= 0 && dlen < kLim && doo >= 0 && doo < kLim)) return nullptr;
+				const size_t vo = (size_t)dvo, len = (size_t)dlen, oo = (size_t)doo, size = buffers[bi].size();
+				if (vo > size || len > size - vo || oo > len || bytes > len - oo) return nullptr;
+				return buffers[bi].data() + vo + oo;
+			}
+
+			// accessor.sparse: count in [1, accessor count], u8 / u16 / u32 indices strictly increasing and below the accessor count,
+			// indices and values (tightly packed, the accessor's element type) inside their views
+			bool Sparse(const Json& s, Accessor& a) const
+			{
+				const double dk = s.at("count").number(0);
+				if (!(dk >= 1.0 && dk <= (double)a.count) || dk != (double)(uint64_t)dk) return false;
+				const size_t k = (size_t)dk;
+				const Json& si = s.at("indices");
+				const int it = si.at("componentType").integer(0);
+				if (it != 5121 && it != 5123 && it != 5125) return false;
+				const uint8_t* at = ViewBytes(si, k * (size_t)CompSize(it));
+				const uint8_t* values = ViewBytes(s.at("values"), k * a.elem);
+				if (!at || !values) return false;
+				for (size_t i = 0; i < k; i++)
+				{
+					const uint32_t v = IndexAt(at, (uint32_t)it, i);
+					if (v >= a.count || (i && v <= IndexAt(at, (uint32_t)it, i - 1))) return false;
+				}
+				a.sparseAt = at; a.sparseValues = values; a.sparseCount = k; a.sparseType = it;
+				return true;
+			}
 		};
 
-		float ReadFloat(const Accessor& a, size_t i, int c)
+		// the bytes of element i (elem of them): a sparse value, the base view's element, or zeros
+		const uint8_t* Element(const Accessor& a, size_t i)
 		{
-			const uint8_t* p = a.base + a.stride * i;
-			switch (a.componentType)
+			static const uint8_t zeros[64] = {};            // the largest element, MAT4 of float
+			size_t lo = 0, hi = a.sparseCount;
+			while (lo < hi)
 			{
-			case 5126: { float v; memcpy(&v, p + 4 * c, 4); return v; }
-			case 5121: { const float v = (float)p[c]; return a.normalized ? v / 255.0f : v; }
-			case 5120: { const float v = (float)((const int8_t*)p)[c]; return a.normalized ? std::max(v / 127.0f, -1.0f) : v; }
-			case 5123: { uint16_t u; memcpy(&u, p + 2 * c, 2); const float v = (float)u; return a.normalized ? v / 65535.0f : v; }
-			case 5122: { int16_t u; memcpy(&u, p + 2 * c, 2); const float v = (float)u; return a.normalized ? std::max(v / 32767.0f, -1.0f) : v; }
-			default: return 0.0f;
+				const size_t mid = (lo + hi) / 2;
+				const uint32_t at = IndexAt(a.sparseAt, (uint32_t)a.sparseType, mid);
+				if (at == i) return a.sparseValues + mid * a.elem;
+				if (at < i) lo = mid + 1; else hi = mid;
 			}
+			return a.base ? a.base + a.stride * i : zeros;
 		}
 
-		uint32_t ReadIndex(const Accessor& a, size_t i)
+		// the first `keep` bytes of every element, tightly packed (the stored form the device reads)
+		void Gather(const Accessor& a, size_t keep, std::vector<uint8_t>& out)
 		{
-			const uint8_t* p = a.base + a.stride * i;
-			switch (a.componentType)
-			{
-			case 5121: return p[0];
-			case 5123: { uint16_t u; memcpy(&u, p, 2); return u; }
-			case 5125: { uint32_t u; memcpy(&u, p, 4); return u; }
-			default: return 0;
-			}
+			out.assign(a.count * keep, 0);
+			if (a.base && a.stride == keep) memcpy(out.data(), a.base, out.size());
+			else if (a.base) for (size_t i = 0; i < a.count; i++) memcpy(out.data() + i * keep, a.base + a.stride * i, keep);
+			for (size_t k = 0; k < a.sparseCount; k++) memcpy(out.data() + (size_t)IndexAt(a.sparseAt, (uint32_t)a.sparseType, k) * keep, a.sparseValues + k * a.elem, keep);
 		}
 
-		void ReadStream(const Accessor& a, int comps, std::vector<float>& out)
+		float ReadFloat(const Accessor& a, size_t i, int c) { return DecodeComponent(Element(a, i), (uint32_t)a.componentType, a.normalized, (uint32_t)c); }
+
+		// an accessor's elements in their stored form, for a vertex stream of the device
+		HostStream Stream(const Accessor& a)
 		{
-			out.resize(a.count * comps);
-			if (a.componentType == 5126 && a.stride == (size_t)comps * 4 && a.comps == comps) { memcpy(out.data(), a.base, out.size() * 4); return; }
-			for (size_t i = 0; i < a.count; i++) for (int c = 0; c < comps; c++) out[i * comps + c] = c < a.comps ? ReadFloat(a, i, c) : 0.0f;
+			HostStream s;
+			Gather(a, a.elem, s.bytes);
+			s.componentType = (uint32_t)a.componentType; s.comps = (uint32_t)a.comps; s.normalized = a.normalized;
+			return s;
 		}
 
 		float ExtNumber(const Json& o, const char* key, float def) { const Json* j = o.find(key); return (j && j->isNumber()) ? (float)j->num : def; }
@@ -352,9 +412,10 @@ namespace spt
 
 			int rc = SAILOR_PT_OK;                 // the first refusal (ERR_FORMAT / ERR_LIMIT) stops the traversal
 			std::string err;
-			// source index by the accessors a primitive reads (POSITION, NORMAL, TANGENT, TEXCOORD_0, TEXCOORD_1, indices): -1 when
-			// the primitive draws nothing
-			std::map<std::array<int, 6>, int> sourceOf;
+			// source index by the accessors a primitive reads (POSITION, NORMAL, TANGENT, TEXCOORD_0, TEXCOORD_1, indices) and its mode:
+			// -1 when the primitive draws nothing
+			std::map<std::array<int, 7>, int> sourceOf;
+			uint64_t numVertices = 0;              // of all sources so far, at most kMaxVertices
 
 			bool Refuse(int code, int node, const std::string& what)
 			{
@@ -395,49 +456,75 @@ namespace spt
 				for (int c = 0; c < 4; c++) for (int r = 0; r < 4; r++) out[c * 4 + r] = m[r * 4 + c]; // transpose
 			}
 
-			// the streams of a primitive, read on its first use; -1 when it draws nothing (not TRIANGLES, POSITION unreadable)
-			int Source(const Json& prim)
+			// the streams of a primitive, read on its first use; -1 when it draws nothing (a mode other than TRIANGLES, TRIANGLE_STRIP
+			// and TRIANGLE_FAN, POSITION unreadable) or when it is refused (rc set: more vertices or faces than a scene may have)
+			int Source(const Json& prim, int node)
 			{
 				const int mode = prim.at("mode").integer(4);
-				if (mode != 4) return -1;
+				if (mode != 4 && mode != 5 && mode != 6) return -1;
 				const Json& attrs = prim.at("attributes");
-				const std::array<int, 6> key = { attrs.at("POSITION").integer(-1), attrs.at("NORMAL").integer(-1), attrs.at("TANGENT").integer(-1),
-					attrs.at("TEXCOORD_0").integer(-1), attrs.at("TEXCOORD_1").integer(-1), prim.at("indices").integer(-1) };
+				const std::array<int, 7> key = { attrs.at("POSITION").integer(-1), attrs.at("NORMAL").integer(-1), attrs.at("TANGENT").integer(-1),
+					attrs.at("TEXCOORD_0").integer(-1), attrs.at("TEXCOORD_1").integer(-1), prim.at("indices").integer(-1), mode };
 				const auto found = sourceOf.find(key);
 				if (found != sourceOf.end()) return found->second;
 				int& slot = sourceOf[key];
 				slot = -1;
 				const Accessor pos = g.accessor(key[0]);
 				if (!pos.valid) return -1;
+				const Accessor idx = g.accessor(key[5]);
+				// the counts come from the file (a sparse accessor without a bufferView is not bounded by the file's size): each passes
+				// the limit of its consumer before anything is sized by it
+				const uint64_t n = idx.valid ? idx.count : pos.count;
+				const uint64_t faces = mode == 4 ? n / 3 : (n > 2 ? n - 2 : 0);
+				if (pos.count > kMaxVertices - numVertices) { Refuse(SAILOR_PT_ERR_LIMIT, node, "the scene has more than " + std::to_string(kMaxVertices) + " vertices"); return -1; }
+				if (faces > kMaxTriangles) { Refuse(SAILOR_PT_ERR_LIMIT, node, "a primitive has more than " + std::to_string(kMaxTriangles) + " triangles"); return -1; }
+				numVertices += pos.count;
 				scene.sources.emplace_back();
 				HostSource& hp = scene.sources.back();
 				slot = (int)scene.sources.size() - 1;
-				ReadStream(pos, 3, hp.pos);
+				hp.numVerts = pos.count; hp.mode = (uint32_t)mode; hp.faces = faces;
+				hp.pos = Stream(pos);
 				// an attribute stream whose element count differs from POSITION's is malformed: it is ignored (the device buffers are
 				// sized by the position count, and FlattenKernel indexes every stream with position indices)
 				auto attr = [&](int k) { Accessor a = g.accessor(key[k]); if (a.valid && a.count != pos.count) a.valid = false; return a; };
 				const Accessor nrm = attr(1);
-				if (nrm.valid) ReadStream(nrm, 3, hp.nrm);
+				if (nrm.valid) hp.nrm = Stream(nrm);
 				const Accessor tan = attr(2);
-				if (tan.valid && tan.comps == 4) ReadStream(tan, 4, hp.tan);
+				if (tan.valid && tan.comps == 4) hp.tan = Stream(tan);
 				const Accessor uv0 = attr(3);
-				if (uv0.valid) ReadStream(uv0, 2, hp.uv0);
+				if (uv0.valid) hp.uv0 = Stream(uv0);
 				const Accessor uv1 = attr(4);
-				if (uv1.valid) ReadStream(uv1, 2, hp.uv1);
-				const Accessor idx = g.accessor(key[5]);
-				const size_t numIdx = idx.valid ? idx.count : pos.count;
-				const size_t faces = numIdx / 3;
-				hp.idx.resize(faces * 3);
-				uint32_t* dst = hp.idx.data();
-				const size_t n3 = faces * 3;
-				// tightly packed index buffers (what every exporter writes) are converted by typed loops the compiler vectorises; the
-				// per-element switch of ReadIndex cost ~10 ms per million triangles
-				if (idx.valid && idx.componentType == 5125 && idx.stride == 4) memcpy(dst, idx.base, n3 * 4);
-				else if (idx.valid && idx.componentType == 5123 && idx.stride == 2) { for (size_t i = 0; i < n3; i++) { uint16_t u; memcpy(&u, idx.base + 2 * i, 2); dst[i] = u; } }
-				else if (idx.valid && idx.componentType == 5121 && idx.stride == 1) { for (size_t i = 0; i < n3; i++) dst[i] = idx.base[i]; }
-				else for (size_t i = 0; i < n3; i++) dst[i] = idx.valid ? ReadIndex(idx, i) : (uint32_t)i;
+				if (uv1.valid) hp.uv1 = Stream(uv1);
+				if (!idx.valid) return slot;                     // not indexed: AssembleIndexKernel numbers the vertices
+				hp.idxType = (uint32_t)idx.componentType;
+				const size_t cs = (size_t)CompSize(idx.componentType);
+				const bool packed = idx.base && idx.stride == cs && !idx.sparseCount;       // what exporters write: read in place
+				const bool typed = hp.idxType == 5121 || hp.idxType == 5123 || hp.idxType == 5125;
+				const bool list = mode == 4 && typed && (hp.idxType == 5125 || hp.FloatStreams());
+				if (!packed) Gather(idx, cs, hp.idx);
+				else if (!list) hp.idx.assign(idx.base, idx.base + idx.count * cs);
+				if (!list) return slot;
+				// A TRIANGLES list of u32 indices, or of u8 / u16 indices in a source of float32 streams, goes to the device as u32
+				// triples that FlattenKernel reads in place (so files of float32 streams upload what they always did).  Out-of-range
+				// indices read vertex 0 (no crash on bad files), as AssembleIndexKernel does for every other index form.  Typed loops:
+				// the compiler vectorises them (a per-element switch cost ~10 ms per million triangles).
+				const uint8_t* stored = packed ? idx.base : hp.idx.data();
+				const size_t n3 = (size_t)faces * 3;
+				std::vector<uint8_t> u32(n3 * 4);
 				const uint32_t limit = (uint32_t)(pos.count < 0xFFFFFFFFull ? pos.count : 0xFFFFFFFFull);
-				for (size_t i = 0; i < n3; i++) dst[i] = dst[i] < limit ? dst[i] : 0u;      // out-of-range indices read vertex 0 (no crash on bad files)
+				auto widen = [&](auto zero)
+					{
+						using T = decltype(zero);
+						for (size_t i = 0; i < n3; i++)
+						{
+							T v; memcpy(&v, stored + sizeof(T) * i, sizeof(T));
+							const uint32_t c = (uint32_t)v < limit ? (uint32_t)v : 0u;
+							memcpy(u32.data() + 4 * i, &c, 4);
+						}
+					};
+				if (hp.idxType == 5121) widen(uint8_t(0)); else if (hp.idxType == 5123) widen(uint16_t(0)); else widen(uint32_t(0));
+				hp.idx.swap(u32);
+				hp.idxType = 5125;
 				return slot;
 			}
 
@@ -460,7 +547,7 @@ namespace spt
 					{
 						if (src[i] < 0) continue;
 						const uint32_t material = Material(prims.at(i));
-						const uint64_t faces = scene.sources[(size_t)src[i]].idx.size() / 3;
+						const uint64_t faces = scene.sources[(size_t)src[i]].faces;
 						if (!faces) continue;
 						scene.draws.emplace_back();
 						HostDraw& d = scene.draws.back();
@@ -492,6 +579,9 @@ namespace spt
 				if (meshFaces && (uint64_t)count > (kMaxTriangles - scene.numTriangles) / meshFaces)
 					return Refuse(SAILOR_PT_ERR_LIMIT, node, "EXT_mesh_gpu_instancing: " + std::to_string(count) + " instances of " + std::to_string(meshFaces) +
 						" triangles exceed the " + std::to_string(kMaxTriangles) + " triangles a scene may have");
+				// a mesh that draws nothing gets no per-instance data: its count has passed no bound (a sparse accessor without a
+				// bufferView can claim any count below 1e15)
+				if (!meshFaces) return true;
 				out.resize(count * 16);
 				for (size_t i = 0; i < count; i++)
 				{
@@ -519,7 +609,8 @@ namespace spt
 					const Json& prims = g.root.at("meshes").at(mesh).at("primitives");
 					std::vector<int> src(prims.size());
 					uint64_t faces = 0;
-					for (size_t i = 0; i < prims.size(); i++) { src[i] = Source(prims.at(i)); if (src[i] >= 0) faces += scene.sources[(size_t)src[i]].idx.size() / 3; }
+					for (size_t i = 0; i < prims.size(); i++) { src[i] = Source(prims.at(i), index); if (src[i] >= 0) faces += scene.sources[(size_t)src[i]].faces; }
+					if (rc != SAILOR_PT_OK) return;
 					const Json* inst = n.at("extensions").find("EXT_mesh_gpu_instancing");
 					if (inst && inst->find("attributes"))
 					{
@@ -591,7 +682,18 @@ namespace spt
 		};
 	}
 
+	static int LoadGltfFile(const char* path, HostScene& scene, std::string& err);
+
+	// Every count that sizes an allocation is bounded first, but a bounded scene can still need more host memory than there is: that is
+	// an error code, not an exception crossing the C ABI.
 	int LoadGltf(const char* path, HostScene& scene, std::string& err)
+	{
+		try { return LoadGltfFile(path, scene, err); }
+		catch (const std::bad_alloc&) { scene = HostScene(); err = "the scene needs more host memory than is available"; return SAILOR_PT_ERR_LIMIT; }
+		catch (const std::length_error&) { scene = HostScene(); err = "the scene needs more host memory than is available"; return SAILOR_PT_ERR_LIMIT; }
+	}
+
+	static int LoadGltfFile(const char* path, HostScene& scene, std::string& err)
 	{
 		MappedFile file;
 		const std::string p = path;

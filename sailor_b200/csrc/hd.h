@@ -10,6 +10,7 @@
 #include <stdint.h>
 #include <math.h>
 #include <float.h>
+#include <string.h>
 
 #if defined(__CUDACC__)
 #define SPT_HD __host__ __device__ __forceinline__
@@ -96,6 +97,45 @@ namespace spt
 	struct U4 { uint32_t x, y, z, w; };
 	inline U4 ld4u(const void* p) { return *reinterpret_cast<const U4*>(p); }
 #endif
+
+	// A scalar of a glTF buffer: an aligned load on the device (staged streams start at multiples of 4 bytes), memcpy on the host
+	// (an accessor inside a file need not be aligned)
+	template<class T> SPT_HD T load_as(const uint8_t* p)
+	{
+#if defined(__CUDA_ARCH__)
+		return *reinterpret_cast<const T*>(p);
+#else
+		T v; memcpy(&v, p, sizeof(T)); return v;
+#endif
+	}
+
+	// Component c of a stored vertex-attribute element as float (glTF 2.0 accessors, KHR_mesh_quantization): u8 v/255, u16 v/65535,
+	// i8 max(v/127, -1), i16 max(v/32767, -1) when normalized, (float)v otherwise; u32 and unknown component types read 0.  The
+	// loader (instance TRS) and DecodeStreamKernel (vertex streams) both decode through here, so both give the same bits.
+	SPT_HD float DecodeComponent(const uint8_t* e, uint32_t componentType, bool normalized, uint32_t c)
+	{
+		switch (componentType)
+		{
+		case 5126: return load_as<float>(e + 4 * c);
+		case 5121: { const float v = (float)e[c]; return normalized ? v / 255.0f : v; }
+		case 5120: { const float v = (float)load_as<int8_t>(e + c); return normalized ? std_max(v / 127.0f, -1.0f) : v; }
+		case 5123: { const float v = (float)load_as<uint16_t>(e + 2 * c); return normalized ? v / 65535.0f : v; }
+		case 5122: { const float v = (float)load_as<int16_t>(e + 2 * c); return normalized ? std_max(v / 32767.0f, -1.0f) : v; }
+		default: return 0.0f;
+		}
+	}
+
+	// Entry i of a stored index list (u8 / u16 / u32; any other component type reads 0)
+	SPT_HD uint32_t IndexAt(const uint8_t* p, uint32_t componentType, uint64_t i)
+	{
+		switch (componentType)
+		{
+		case 5121: return p[i];
+		case 5123: return load_as<uint16_t>(p + 2 * i);
+		case 5125: return load_as<uint32_t>(p + 4 * i);
+		default: return 0u;
+		}
+	}
 
 	// Reference constants
 	constexpr float kPiSailor = 3.1415926f;            // Math::Pi (Runtime/Math/Math.h:14)

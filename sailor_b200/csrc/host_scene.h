@@ -27,16 +27,37 @@ namespace spt
 	};
 	static_assert(sizeof(MaterialGpu) == 144, "MaterialGpu layout");
 
-	// The vertex streams of one glTF primitive, read once per document: every node that reaches a primitive with the same
-	// accessors, and every instance of EXT_mesh_gpu_instancing, draws these streams again without copying them.
+	// One vertex stream as the file stores it (sparse substitution applied): one element per vertex of `comps` components of
+	// `componentType`, tightly packed.  The device decodes it (DecodeComponent, hd.h) unless it already is the float32 stream
+	// FlattenKernel reads.
+	struct HostStream
+	{
+		std::vector<uint8_t> bytes;     // empty: the primitive has no such stream
+		uint32_t componentType = 0, comps = 0;
+		bool normalized = false;
+		bool empty() const { return bytes.empty(); }
+		bool IsFloat(uint32_t width) const { return componentType == 5126 && comps == width; }
+	};
+
+	// The streams of one glTF primitive, read once per document: every node that reaches a primitive with the same accessors
+	// and mode, and every instance of EXT_mesh_gpu_instancing, draws these streams again without copying them.
 	struct HostSource
 	{
-		std::vector<float> pos;     // 3 per vertex
-		std::vector<float> nrm;     // 3 per vertex or empty (-> flat face normals, aiProcess_GenNormals)
-		std::vector<float> uv0;     // 2 per vertex or empty
-		std::vector<float> uv1;     // 2 per vertex or empty
-		std::vector<float> tan;     // 4 per vertex or empty
-		std::vector<uint32_t> idx;  // 3 per triangle (identity when the primitive is not indexed)
+		uint64_t numVerts = 0;
+		HostStream pos;             // decoded to 3 floats per vertex
+		HostStream nrm;             // 3 or empty (-> flat face normals, aiProcess_GenNormals)
+		HostStream uv0, uv1;        // 2 or empty
+		HostStream tan;             // 4 (a VEC4 accessor) or empty
+		uint32_t mode = 4;          // 4 TRIANGLES, 5 TRIANGLE_STRIP, 6 TRIANGLE_FAN
+		uint32_t idxType = 0;       // component type of `idx`; 0: not indexed (the vertices in order)
+		std::vector<uint8_t> idx;   // the index accessor's first components as stored, tightly packed; a u32 TRIANGLES list is clamped
+		uint64_t faces = 0;         // TRIANGLES n / 3, strip and fan max(n - 2, 0); n = index count, or numVerts without indices
+		// u32 triples that go to the device as they are (every other index form is assembled there by AssembleIndexKernel)
+		bool DirectIdx() const { return mode == 4 && idxType == 5125; }
+		bool FloatStreams() const
+		{
+			return pos.IsFloat(3) && (nrm.empty() || nrm.IsFloat(3)) && (uv0.empty() || uv0.IsFloat(2)) && (uv1.empty() || uv1.IsFloat(2)) && (tan.empty() || tan.IsFloat(4));
+		}
 	};
 
 	// One placement of a source in the flattened scene.  Draws are in the scene's triangle order: the flattened triangles are
@@ -53,6 +74,8 @@ namespace spt
 	// node indices stay below 2 N and leaf references below 2^31 (traverse.cuh kLeafBit).  floor((2^32 - 1) / 3) keeps all of
 	// them exact.  Device memory runs out long before this (about 232 B per flattened triangle plus the BVH).
 	constexpr uint64_t kMaxTriangles = 0xFFFFFFFFull / 3u;
+	// Most vertices all sources of a scene may have together: FlattenKernel forms vertex * 4 (tangents) in 32 bits.
+	constexpr uint64_t kMaxVertices = 0xFFFFFFFFull / 4u;
 
 	struct HostTexture
 	{

@@ -162,25 +162,48 @@ namespace spt
 			numTris = (uint32_t)H.numTriangles;
 			counter.Alloc(ctx, 16); counter.Zero(ctx);
 			if (numTris == 0) return CudaStatus();
-			// Each source primitive's streams go to the device once, however many draws place it.  With few sources they are copied
-			// piece by piece, straight from the importer's vectors (no host-side concatenation: at 10 M triangles that was hundreds of
-			// MB of extra copies).  A stream a source lacks is never read (FlattenKernel looks at SourceDesc::has*), so its part of
-			// the device buffer stays uninitialised.
+			// Each source primitive's streams go to the device once, however many draws place it.  A float32 stream of the width
+			// FlattenKernel reads and a u32 TRIANGLES list go straight into FlattenKernel's buffers.  Every other stream is uploaded as
+			// the file stores it and decoded in place by DecodeStreamKernel; every other index form (u8 / u16 indices of quantized
+			// sources, strips, fans, no indices) is turned into u32 triples by AssembleIndexKernel.  A stream a source lacks is never
+			// read (FlattenKernel looks at SourceDesc::has*), so its part of the device buffer stays uninitialised.
+			constexpr int kKinds = 5;                                     // pos, nrm, uv0, uv1, tan
+			const uint32_t width[kKinds] = { 3, 3, 2, 2, 4 };
+			auto streamOf = [](const HostSource& hs, int k) -> const HostStream& { return k == 0 ? hs.pos : k == 1 ? hs.nrm : k == 2 ? hs.uv0 : k == 3 ? hs.uv1 : hs.tan; };
+			auto align4 = [](uint64_t b) { return (b + 3u) & ~(uint64_t)3u; };
 			std::vector<SourceDesc> srcs(H.sources.size());
-			uint64_t vtxTotal = 0, idxTotal = 0;
-			bool anyNrm = false, anyUv0 = false, anyUv1 = false, anyTan = false;
+			std::vector<StreamDecodeDesc> dec[kKinds]; std::vector<uint32_t> decStart[kKinds];
+			std::vector<IndexAssemblyDesc> asmb; std::vector<uint32_t> asmStart;
+			uint64_t vtxTotal = 0, idxTotal = 0, decVerts[kKinds] = {}, staged[kKinds + 1] = {}, asmFaces = 0;     // staged[kKinds]: indices
+			bool any[kKinds] = {};
 			for (size_t i = 0; i < H.sources.size(); i++)
 			{
 				const HostSource& hs = H.sources[i];
 				SourceDesc& d = srcs[i];
 				memset(&d, 0, sizeof(d));
 				d.vtxOffset = (uint32_t)vtxTotal; d.idxOffset = (uint32_t)idxTotal;
-				d.hasNrm = !hs.nrm.empty(); d.hasUv0 = !hs.uv0.empty(); d.hasUv1 = !hs.uv1.empty(); d.hasTan = !hs.tan.empty();
-				anyNrm |= d.hasNrm != 0; anyUv0 |= d.hasUv0 != 0; anyUv1 |= d.hasUv1 != 0; anyTan |= d.hasTan != 0;
-				vtxTotal += hs.pos.size() / 3; idxTotal += hs.idx.size();
+				uint32_t* has[kKinds] = { nullptr, &d.hasNrm, &d.hasUv0, &d.hasUv1, &d.hasTan };
+				for (int k = 0; k < kKinds; k++)
+				{
+					const HostStream& st = streamOf(hs, k);
+					if (st.empty()) continue;
+					if (has[k]) *has[k] = 1;
+					any[k] = true;
+					if (st.IsFloat(width[k])) continue;
+					decStart[k].push_back((uint32_t)decVerts[k]);
+					dec[k].push_back(StreamDecodeDesc{ staged[k], (uint32_t)vtxTotal, st.componentType, st.comps, st.normalized ? 1u : 0u, { 0, 0 } });
+					decVerts[k] += hs.numVerts; staged[k] += align4(st.bytes.size());
+				}
+				if (!hs.DirectIdx() && hs.faces)
+				{
+					asmStart.push_back((uint32_t)asmFaces);
+					asmb.push_back(IndexAssemblyDesc{ staged[kKinds], (uint32_t)idxTotal, hs.idxType, hs.mode, (uint32_t)hs.numVerts, { 0, 0 } });
+					asmFaces += hs.faces; staged[kKinds] += align4(hs.idx.size());
+				}
+				vtxTotal += hs.numVerts; idxTotal += hs.faces * 3;
 			}
 			// FlattenKernel forms vertex * 4 (tangents) and index offsets in 32 bits
-			if (vtxTotal > 0xFFFFFFFFull / 4u || idxTotal > 0xFFFFFFFFull) { ctx.error = "the scene's vertex streams are too large for 32-bit offsets"; return SAILOR_PT_ERR_LIMIT; }
+			if (vtxTotal > kMaxVertices || idxTotal > 0xFFFFFFFFull) { ctx.error = "the scene's vertex streams are too large for 32-bit offsets"; return SAILOR_PT_ERR_LIMIT; }
 			const uint32_t vtxOffset = (uint32_t)vtxTotal, idxOffset = (uint32_t)idxTotal;
 			std::vector<DrawDesc> draws(H.draws.size());
 			std::vector<uint32_t> drawStart(H.draws.size() + 1);
@@ -193,63 +216,78 @@ namespace spt
 				memcpy(d.world, hd.world, sizeof(d.world));
 				d.source = hd.source; d.material = hd.material;
 				drawStart[i] = (uint32_t)triStart;
-				triStart += H.sources[hd.source].idx.size() / 3;
+				triStart += H.sources[hd.source].faces;
 			}
 			drawStart[H.draws.size()] = (uint32_t)triStart;
 			if (triStart != numTris) { ctx.error = "draw table does not cover the scene's triangles"; return SAILOR_PT_ERR_FORMAT; }
 
 			DevBuf<SourceDesc> dSrcs; DevBuf<DrawDesc> dDraws; DevBuf<uint32_t> dDrawStart, dBlockDraw;
-			DevBuf<float> dPos, dNrm, dUv0, dUv1, dTan; DevBuf<uint32_t> dIdx;
+			DevBuf<float> dStream[kKinds]; DevBuf<uint32_t> dIdx;
+			// staging of the stored forms and their tables: freed when Upload returns, behind the flatten pass on the stream
+			DevBuf<uint8_t> dStaged[kKinds + 1]; DevBuf<StreamDecodeDesc> dDec[kKinds]; DevBuf<uint32_t> dDecStart[kKinds], dAsmStart; DevBuf<IndexAssemblyDesc> dAsm;
 			dSrcs.Upload(ctx, srcs); dDraws.Upload(ctx, draws); dDrawStart.Upload(ctx, drawStart);
 			const uint32_t numBlocks = (numTris - 1u) / kFlattenSpan + 1u;
 			dBlockDraw.Alloc(ctx, (size_t)numBlocks + 1);
-			dPos.Alloc(ctx, (size_t)vtxOffset * 3 + 1); dIdx.Alloc(ctx, (size_t)idxOffset + 1);
-			dNrm.Alloc(ctx, anyNrm ? (size_t)vtxOffset * 3 : 1); dUv0.Alloc(ctx, anyUv0 ? (size_t)vtxOffset * 2 : 1);
-			dUv1.Alloc(ctx, anyUv1 ? (size_t)vtxOffset * 2 : 1); dTan.Alloc(ctx, anyTan ? (size_t)vtxOffset * 4 : 1);
-			if (!ctx.ok) return CudaStatus();
-			if (H.sources.size() > 32)
+			dIdx.Alloc(ctx, (size_t)idxOffset + 1);
+			for (int k = 0; k < kKinds; k++)
 			{
-				// many small sources: one copy per stream from a host-side concatenation beats thousands of tiny transfers
-				std::vector<float> pos((size_t)vtxOffset * 3), nrm(anyNrm ? (size_t)vtxOffset * 3 : 0), uv0(anyUv0 ? (size_t)vtxOffset * 2 : 0), uv1(anyUv1 ? (size_t)vtxOffset * 2 : 0), tan(anyTan ? (size_t)vtxOffset * 4 : 0);
-				std::vector<uint32_t> idx(idxOffset);
+				dStream[k].Alloc(ctx, k == 0 ? (size_t)vtxOffset * 3 + 1 : (any[k] ? (size_t)vtxOffset * width[k] : 1));
+				if (staged[k]) { dStaged[k].Alloc(ctx, staged[k]); dDec[k].Upload(ctx, dec[k]); dDecStart[k].Upload(ctx, decStart[k]); }
+			}
+			if (staged[kKinds]) dStaged[kKinds].Alloc(ctx, staged[kKinds]);
+			if (!asmb.empty()) { dAsm.Upload(ctx, asmb); dAsmStart.Upload(ctx, asmStart); }
+			if (!ctx.ok) return CudaStatus();
+			{
+				// With few sources the pieces are copied one by one, straight from the importer's vectors (no host-side concatenation:
+				// at 10 M triangles that was hundreds of MB of extra copies); with many, one copy per buffer of a host-side concatenation
+				// beats thousands of tiny transfers.
+				const bool concat = H.sources.size() > 32;
+				struct Pieces
+				{
+					uint8_t* dev; bool concat; std::vector<uint8_t> host; size_t lo = ~(size_t)0, hi = 0;
+					void Put(Ctx& ctx, size_t off, const void* src, size_t bytes)
+					{
+						if (!bytes) return;
+						if (!concat) { DevUpload(ctx, dev + off, src, bytes); return; }
+						if (host.size() < off + bytes) host.resize(off + bytes);
+						memcpy(host.data() + off, src, bytes);
+						lo = off < lo ? off : lo; hi = off + bytes > hi ? off + bytes : hi;
+					}
+					void Flush(Ctx& ctx) { if (hi > lo) DevUpload(ctx, dev + lo, host.data() + lo, hi - lo); }
+				};
+				std::vector<Pieces> direct, stage;
+				for (int k = 0; k < kKinds; k++) direct.push_back(Pieces{ (uint8_t*)dStream[k].p, concat }), stage.push_back(Pieces{ dStaged[k].p, concat });
+				direct.push_back(Pieces{ (uint8_t*)dIdx.p, concat }); stage.push_back(Pieces{ dStaged[kKinds].p, concat });
+				uint64_t off[kKinds + 1] = {};
 				for (size_t i = 0; i < H.sources.size(); i++)
 				{
 					const HostSource& hs = H.sources[i];
 					const SourceDesc& d = srcs[i];
-					if (!hs.pos.empty()) memcpy(pos.data() + (size_t)d.vtxOffset * 3, hs.pos.data(), hs.pos.size() * sizeof(float));
-					if (!hs.idx.empty()) memcpy(idx.data() + d.idxOffset, hs.idx.data(), hs.idx.size() * sizeof(uint32_t));
-					if (d.hasNrm) memcpy(nrm.data() + (size_t)d.vtxOffset * 3, hs.nrm.data(), hs.nrm.size() * sizeof(float));
-					if (d.hasUv0) memcpy(uv0.data() + (size_t)d.vtxOffset * 2, hs.uv0.data(), hs.uv0.size() * sizeof(float));
-					if (d.hasUv1) memcpy(uv1.data() + (size_t)d.vtxOffset * 2, hs.uv1.data(), hs.uv1.size() * sizeof(float));
-					if (d.hasTan) memcpy(tan.data() + (size_t)d.vtxOffset * 4, hs.tan.data(), hs.tan.size() * sizeof(float));
+					for (int k = 0; k < kKinds; k++)
+					{
+						const HostStream& st = streamOf(hs, k);
+						if (st.empty()) continue;
+						if (st.IsFloat(width[k])) direct[k].Put(ctx, (size_t)d.vtxOffset * width[k] * sizeof(float), st.bytes.data(), st.bytes.size());
+						else { stage[k].Put(ctx, off[k], st.bytes.data(), st.bytes.size()); off[k] += align4(st.bytes.size()); }
+					}
+					if (hs.DirectIdx()) direct[kKinds].Put(ctx, (size_t)d.idxOffset * sizeof(uint32_t), hs.idx.data(), (size_t)hs.faces * 3 * sizeof(uint32_t));
+					else if (hs.faces) { stage[kKinds].Put(ctx, off[kKinds], hs.idx.data(), hs.idx.size()); off[kKinds] += align4(hs.idx.size()); }
 				}
-				if (!pos.empty()) DevUpload(ctx, dPos.p, pos.data(), pos.size() * sizeof(float));
-				if (!idx.empty()) DevUpload(ctx, dIdx.p, idx.data(), idx.size() * sizeof(uint32_t));
-				if (!nrm.empty()) DevUpload(ctx, dNrm.p, nrm.data(), nrm.size() * sizeof(float));
-				if (!uv0.empty()) DevUpload(ctx, dUv0.p, uv0.data(), uv0.size() * sizeof(float));
-				if (!uv1.empty()) DevUpload(ctx, dUv1.p, uv1.data(), uv1.size() * sizeof(float));
-				if (!tan.empty()) DevUpload(ctx, dTan.p, tan.data(), tan.size() * sizeof(float));
-				ctx.Sync();                                   // the staging vectors die at the end of this block
-			}
-			else for (size_t i = 0; i < H.sources.size(); i++)
-			{
-				const HostSource& hs = H.sources[i];
-				const SourceDesc& d = srcs[i];
-				if (!hs.pos.empty()) DevUpload(ctx, dPos.p + (size_t)d.vtxOffset * 3, hs.pos.data(), hs.pos.size() * sizeof(float));
-				if (!hs.idx.empty()) DevUpload(ctx, dIdx.p + d.idxOffset, hs.idx.data(), hs.idx.size() * sizeof(uint32_t));
-				if (d.hasNrm) DevUpload(ctx, dNrm.p + (size_t)d.vtxOffset * 3, hs.nrm.data(), hs.nrm.size() * sizeof(float));
-				if (d.hasUv0) DevUpload(ctx, dUv0.p + (size_t)d.vtxOffset * 2, hs.uv0.data(), hs.uv0.size() * sizeof(float));
-				if (d.hasUv1) DevUpload(ctx, dUv1.p + (size_t)d.vtxOffset * 2, hs.uv1.data(), hs.uv1.size() * sizeof(float));
-				if (d.hasTan) DevUpload(ctx, dTan.p + (size_t)d.vtxOffset * 4, hs.tan.data(), hs.tan.size() * sizeof(float));
+				for (int k = 0; k <= kKinds; k++) { direct[k].Flush(ctx); stage[k].Flush(ctx); }
+				if (concat) ctx.Sync();                       // the staging vectors die at the end of this block
 			}
 			vtx.Alloc(ctx, (size_t)numTris * 3); centroid.Alloc(ctx, numTris); shade.Alloc(ctx, (size_t)numTris * 9); uv2.Alloc(ctx, (size_t)numTris * 3);
 			if (!ctx.ok) return CudaStatus();
 
+			// secondsFlatten: the decode and assembly passes (none for files of float32 streams and u32 lists) and the flatten pass
 			ctx.TimerStart();
+			for (int k = 0; k < kKinds; k++)
+				if (decVerts[k]) launch_for(ctx, (uint32_t)decVerts[k], DecodeStreamKernel{ dDecStart[k].p, dDec[k].p, (uint32_t)dec[k].size(), width[k], dStaged[k].p, dStream[k].p });
+			if (asmFaces) launch_for(ctx, (uint32_t)asmFaces, AssembleIndexKernel{ dAsmStart.p, dAsm.p, (uint32_t)asmb.size(), dStaged[kKinds].p, dIdx.p });
 			launch_for(ctx, numBlocks + 1u, FlattenBlockKernel{ dDrawStart.p, (uint32_t)draws.size(), numTris, dBlockDraw.p });
 			FlattenKernel fk;
 			fk.draws = dDraws.p; fk.drawStart = dDrawStart.p; fk.blockDraw = dBlockDraw.p; fk.sources = dSrcs.p;
-			fk.pos = dPos.p; fk.nrm = dNrm.p; fk.uv0 = dUv0.p; fk.uv1 = dUv1.p; fk.tan = dTan.p; fk.idx = dIdx.p;
+			fk.pos = dStream[0].p; fk.nrm = dStream[1].p; fk.uv0 = dStream[2].p; fk.uv1 = dStream[3].p; fk.tan = dStream[4].p; fk.idx = dIdx.p;
 			fk.vtx = vtx.p; fk.centroid = centroid.p; fk.shade = shade.p; fk.uv2 = uv2.p;
 			launch_for(ctx, numTris, fk);
 			stats.secondsFlatten = ctx.TimerStop();
